@@ -7,10 +7,14 @@ setEigenDecomposition, setCategoryRates/Weights, setStateFrequencies, updateTran
 (2N-2 branches), updatePartials (N-1 operations), calculateRootLogLikelihoods -- through the C ABI
 of libhmsbeagle.so, with BEAST's double-buffer index flipping between steps.
 
-  value : K steps enqueued back to back on the instance stream (tip data / partials resident in HBM, result left on
-          the device), bracketed by barrier + synchronize, CUDA-event timed on the engine's stream, max over ranks.
-          The K-step block is repeated (>= 25 times, >= ~1 s in total) and the MEDIAN block is reported
-          (`repeats`, `block_ms_p10/p50/p90`): a 20-step block lasts 8 ms and one host hiccup would otherwise be the result.
+  value : exactly K = --steps timed steps enqueued back to back on the instance stream (tip data / partials resident in
+          HBM, result left on the device), bracketed by barrier + synchronize, CUDA-event timed on the engine's stream, max
+          over ranks.  Events split the K steps into `repeats` (up to 25) consecutive windows without a synchronize between
+          them, and the MEDIAN window's per-step time is reported (`block_ms_p10/p50/p90` = K x the per-step quantiles):
+          a host hiccup idles the GPU inside one window only instead of becoming the result.
+  --dump-outputs DIR : after the timed steps, what their last step computed, as a caller receives it: the (joint)
+          log-likelihood (DIR/logL.npy) and the per-pattern site log-likelihoods (DIR/site_logL.npy; one file per rank,
+          site_logL_rank<r>.npy, when N > 1), float64.  The inputs are seeded, so two builds can be compared output for output.
   e2e   : the same sequence through the synchronous reference-facing calls with HOST buffers:
           every step uploads the eigen system, rates, frequencies, branch lengths and op list and
           lands the 8-byte (joint) log-likelihood on the host; median per step, max over ranks.
@@ -31,11 +35,11 @@ from __future__ import annotations
 import argparse
 import ctypes as Cc
 import json
-import math
 import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import time
 
 import numpy as np
@@ -70,6 +74,8 @@ WORKLOADS = {
 }
 FLU8_SITES = [2341, 2341, 2233, 1778, 1565, 1413, 1027, 890]      # SURVEY.md 8d cfg 5: segment-length-like site counts
 
+BENCH_CACHE = os.environ.get("B200_BENCH_CACHE", os.path.join(tempfile.gettempdir(), "b200_bench_cache"))
+
 ZERO = np.zeros(1, dtype=np.int32)
 MINUS1 = np.full(1, -1, dtype=np.int32)
 
@@ -99,8 +105,9 @@ def build_workload(name, shard_index, overrides):
         model = em.SubstitutionModel(rng.uniform(0.2, 3.0, S * (S - 1) // 2), rng.dirichlet(np.full(S, 5.0)))
     site = em.GammaSiteRateModel(shape=0.5, gammaCategoryCount=w["categories"]) if w["categories"] > 1 \
         else em.GammaSiteRateModel()
-    # the simulated alignment is cached per box (sweeps re-use it); it is regenerated when absent
-    cache = os.path.join(os.environ.get("B200_BENCH_CACHE", "/tmp/b200_bench_cache"),
+    # the simulated alignment is cached outside the tree, in the temporary directory (sweeps re-use it); it is regenerated
+    # when absent
+    cache = os.path.join(BENCH_CACHE,
                          f"{w.get('data', name)}_{w['taxa']}_{w['patterns']}_{w['states']}_{w['categories']}_{shard_index}.npz")
     if w.get("fixture"):
         z = np.load(os.path.join(ROOT, "tests", "golden", w["fixture"] + "_patterns.npz"))
@@ -308,6 +315,10 @@ def run_reference_arm(args, meta_base):
         issue_sync(inst, ev, k & 1, out)
         per.append(time.perf_counter() - tc)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        site_logL = np.zeros(P)
+        inst.getSiteLogLikelihoods(site_logL)
+        dump_outputs(args.dump_outputs, float(out[0]), site_logL, 0, 1)
     inst.finalize()
     value = 1.0 / statistics.median(per)        # median step: the same statistic as the cpu_baseline leg of the GPU arm
     line = dict(meta_base)
@@ -384,38 +395,30 @@ def _quantiles(xs):
     return pick(0.10), pick(0.50), pick(0.90)
 
 
-def timed_blocks(D, stream, step_async, steps, warmup, min_repeats=25, min_total_s=1.0, max_repeats=400):
-    """K-step blocks, each bracketed by barrier + synchronize and timed with CUDA events on the engine's stream;
-    per-block max over ranks, then the quantiles over the blocks."""
+def timed_blocks(D, stream, step_async, steps, warmup, windows=25):
+    """Exactly `steps` timed steps after the warm-up, enqueued back to back and bracketed by barrier + synchronize.  CUDA
+    events on the engine's stream split them into up to `windows` consecutive windows of (nearly) equal length; nothing
+    synchronizes between windows, so the GPU never idles at a window boundary.  Per-window max over ranks, then the
+    quantiles of the per-step time over the windows, scaled to the `steps`-step block."""
     torch = D.torch
     for k in range(max(3, warmup)):
         step_async(k)
     D.bracket()
-    # one pilot block decides how many repeats fill ~min_total_s
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record(stream)
-    for k in range(steps):
-        step_async(k)
-    e1.record(stream)
-    D.bracket()
-    pilot = D.max_over_ranks([e0.elapsed_time(e1)])[0]
-    repeats = int(min(max_repeats, max(min_repeats, math.ceil(min_total_s * 1e3 / max(pilot, 1e-3)))))
-    blocks, walls = [], []
-    for _ in range(repeats):
-        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        D.bracket()
-        t0 = time.perf_counter()
-        a.record(stream)
-        for k in range(steps):
+    repeats = max(1, min(windows, steps))
+    bounds = [steps * i // repeats for i in range(repeats + 1)]
+    events = [torch.cuda.Event(enable_timing=True) for _ in range(repeats + 1)]
+    t0 = time.perf_counter()
+    events[0].record(stream)
+    for i in range(repeats):
+        for k in range(bounds[i], bounds[i + 1]):
             step_async(k)
-        b.record(stream)
-        D.bracket()
-        walls.append(time.perf_counter() - t0)
-        blocks.append(a.elapsed_time(b))
-    blocks = D.max_over_ranks(blocks)
-    p10, p50, p90 = _quantiles(blocks)
-    return {"repeats": repeats, "block_ms_p10": p10, "block_ms_p50": p50, "block_ms_p90": p90,
-            "wall_ms_per_step": 1e3 * statistics.median(walls) / steps}
+        events[i + 1].record(stream)
+    D.bracket()
+    wall = time.perf_counter() - t0
+    ms = D.max_over_ranks([events[i].elapsed_time(events[i + 1]) for i in range(repeats)])
+    p10, p50, p90 = _quantiles([m / (bounds[i + 1] - bounds[i]) for i, m in enumerate(ms)])
+    return {"repeats": repeats, "block_ms_p10": steps * p10, "block_ms_p50": steps * p50, "block_ms_p90": steps * p90,
+            "timed_ms": sum(ms), "wall_ms_per_step": 1e3 * wall / steps}
 
 
 def timed_e2e(D, step_e2e, steps):
@@ -478,6 +481,8 @@ def measure_single_partition(D, lib, beagle, w, tree, pats, model, site, steps, 
     # resident eigen system for the asynchronous loop: slot 0 holds it (issue_sync above used parity 0)
     res["blocks"] = timed_blocks(D, stream, step_async, steps, warmup)
     res["joint"] = float(dres.cpu()[0])
+    res["site_logL"] = np.zeros(P)
+    inst.getSiteLogLikelihoods(res["site_logL"])           # the last timed step's root launch wrote them
     if kernel_timing:
         # kernel classes timed live on the engine's stream, in a block of their own (event pairs around every launch)
         D.bracket()
@@ -657,7 +662,7 @@ def strong_makona(D, lib, beagle, steps, warmup):
 def flu8_partitions():
     tree = em.Tree.coalescent(2000, 0.05, 5)
     parts, models, sites = [], [], []
-    cache = os.path.join(os.environ.get("B200_BENCH_CACHE", "/tmp/b200_bench_cache"), "flu8_2000.npz")
+    cache = os.path.join(BENCH_CACHE, "flu8_2000.npz")
     z = np.load(cache, allow_pickle=False) if os.path.exists(cache) else None
     for k, ns in enumerate(FLU8_SITES):
         rng = np.random.default_rng(10 + k)
@@ -745,6 +750,22 @@ def strong_flu8(D, lib, beagle, steps, warmup):
             "logL": e2e["logL"], "steps": steps}
 
 
+MAX_DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, logL, site_logL, rank, world):
+    """Writes the last timed step's results: DIR/logL.npy (rank 0: the joint log-likelihood) and this rank's site
+    log-likelihoods.  Past its share of MAX_DUMP_BYTES a rank writes a fixed seeded sample of its patterns (sorted)."""
+    os.makedirs(path, exist_ok=True)
+    if rank == 0:
+        np.save(os.path.join(path, "logL.npy"), np.array([logL], dtype=np.float64))
+    keep = (MAX_DUMP_BYTES // world - 4096) // 8
+    if site_logL.size > keep:
+        site_logL = site_logL[np.sort(np.random.default_rng(12345).choice(site_logL.size, keep, replace=False))]
+    name = "site_logL.npy" if world == 1 else f"site_logL_rank{rank}.npy"
+    np.save(os.path.join(path, name), np.ascontiguousarray(site_logL, dtype=np.float64))
+
+
 def load_json(path):
     try:
         return json.load(open(path))
@@ -766,6 +787,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the strong-scaling / incremental / cold-plan sections")
     ap.add_argument("--cpu-budget", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's log-likelihood and site "
+                                                          "log-likelihoods to DIR/*.npy")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
@@ -800,6 +823,8 @@ def main():
         sampler.start()
     r = measure_single_partition(D, lib, beagle, w, tree, pats, model, site, args.steps, args.warmup)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r["joint"], r["site_logL"], rank, world)
     ev, inst, S, C, P, out = r["ev"], r["inst"], r["S"], r["C"], r["P"], r["out"]
     scaling = bool(w.get("scaling"))
 
@@ -868,7 +893,9 @@ def main():
         "ms_per_step": dev_ms / args.steps, "wall_ms_per_step": blocks["wall_ms_per_step"],
         "repeats": blocks["repeats"], "block_ms_p10": blocks["block_ms_p10"], "block_ms_p50": blocks["block_ms_p50"],
         "block_ms_p90": blocks["block_ms_p90"],
-        "statistic": "median over `repeats` blocks of `steps` steps, each block = max over ranks of its CUDA-event time",
+        "timed_ms": blocks["timed_ms"],
+        "statistic": "`steps` timed steps in `repeats` consecutive windows, each window = max over ranks of its CUDA-event "
+                     "time; median per-step time over the windows",
         "vs_baseline": None, "logL": r["joint"], "joint_evals_per_s": args.steps / (dev_ms * 1e-3),
         "roofline": roof,
         "e2e": {"value": world / e2e["median_s"], "unit": "evals/s", "ms_per_step": e2e["median_ms"],
